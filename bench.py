@@ -28,6 +28,8 @@ value / e2e / roofline / parity gate / cpu_baseline):
 
 Launch: python bench.py [--gpus N --steps K --warmup W]; for N>1 via torchrun (one rank per GPU).  --scaling weak
 (default): every rank processes its own full-size batch; --scaling strong: the batch is split over the ranks.
+--dump-outputs DIR writes the main workload's records of the last timed step as .npy files; the inputs are seeded, so two
+builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -46,6 +48,7 @@ sys.path.insert(0, ROOT)
 DEFAULT_READS = {'endtrim': 1000000, 'demux': 1000000, 'middle': 1250000, 'sweep': 0}
 SWEEP_LENGTHS = '500,1000,2000,5000,10000,20000,50000,100000'
 OUT_CAP_BYTES = 320 << 20          # e2e: records copied back per call (larger batches go through the ABI in read chunks)
+DUMP_CAP_BYTES = 60000000          # --dump-outputs: all files together stay below 64 MB
 
 
 def parse_args():
@@ -69,6 +72,10 @@ def parse_args():
                          'device, 4 + 4*adapters bytes per window come back instead of 36 per alignment')
     ap.add_argument('--opt', action='append', default=[], metavar='NAME=VALUE',
                     help='engine option for this run (pb200SetOption), e.g. --opt scratch_mb=72')
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='write the records of the last timed step of the main workload to DIR/*.npy (float64, at most '
+                         '%d MB in all: a fixed seeded sample of rows where larger), to compare two builds output for output'
+                         % (DUMP_CAP_BYTES // 1000000))
     return ap.parse_args()
 
 
@@ -650,6 +657,23 @@ def measure_gpu(workload, args, ctx, K, Wm, main):
     return line, res
 
 
+def dump_outputs(out_dir, workload, dev):
+    """The 9-int records the timed device-resident path left in its output buffers after its last step, one pair of
+    float64 files per batch: <workload>_<batch>_records.npy [rows, 9] and <workload>_<batch>_rows.npy (the pair index of
+    each row).  A batch larger than its share of DUMP_CAP_BYTES keeps a sample of rows drawn with a fixed seed."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    keep = DUMP_CAP_BYTES // len(dev) // (10 * 8)
+    for (name, _, _, _), d in zip(workload.batches, dev):
+        rec = d[4]
+        n = rec.shape[0]
+        rows = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        sel = rec.index_select(0, torch.from_numpy(rows).to(rec.device)).cpu().numpy()
+        base = os.path.join(out_dir, '%s_%s' % (workload.name, name))
+        np.save(base + '_records.npy', sel.astype(np.float64))
+        np.save(base + '_rows.npy', rows.astype(np.float64))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -685,6 +709,8 @@ def run_b200(args):
     def one(name, K, Wm, main):
         w = make_workload(name, args, rank, world, main, alloc=alloc)
         line, res = measure_gpu(w, args, ctx, K, Wm, main)
+        if main and rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, w, res['dev'])
         if rank == 0 and world == 1 and not args.no_cpu_baseline:
             try:
                 os.sched_setaffinity(0, all_cpus)          # the CPU baseline runs on ALL host cores, not the GPU's NUMA node

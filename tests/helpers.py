@@ -10,6 +10,22 @@ GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 DEFAULT = [3, -6, -5, -2]
 
 
+def porechop_checkout():
+    """A checkout of rrwick/Porechop (its Python package and test fixtures), which the tests that run its CLI need and
+    skip without: $PORECHOP_CHECKOUT, else the checkout oracle/_ref was built from (oracle/Makefile `ref`), else ''."""
+    path = os.environ.get('PORECHOP_CHECKOUT', '')
+    if not path:
+        try:
+            with open(os.path.join(ROOT, 'oracle', '_ref', 'checkout')) as f:
+                path = f.read().strip()
+        except OSError:
+            pass
+    return path if path and os.path.isdir(path) else ''
+
+
+PORECHOP_CHECKOUT = porechop_checkout()
+
+
 class Rec(ctypes.Structure):
     _fields_ = [('v', ctypes.c_int32 * 9)]
 

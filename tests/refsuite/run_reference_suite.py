@@ -66,11 +66,17 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--modes', default='reference,patch,flat')
     ap.add_argument('--engine', default='oracle', choices=['oracle', 'sim', 'cuda'])
-    ap.add_argument('--ref', default='/root/reference')
+    ap.add_argument('--ref', default='', help='Porechop checkout (default: tests/helpers.py porechop_checkout())')
     ap.add_argument('-k', default='')
     ap.add_argument('--jobs', type=int, default=max(1, (os.cpu_count() or 2) // 2))
     ap.add_argument('--json', default='')
     a = ap.parse_args()
+    if not a.ref:
+        sys.path.insert(0, os.path.dirname(HERE))
+        from helpers import porechop_checkout
+        a.ref = porechop_checkout()
+        if not a.ref:
+            sys.exit('no Porechop checkout: pass --ref or set PORECHOP_CHECKOUT')
     out = {}
     for mode in a.modes.split(','):
         out[mode] = run_mode(mode, a.engine, a.ref, a.k, a.jobs)

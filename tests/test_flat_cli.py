@@ -3,7 +3,7 @@
 Both run in-process on the reference's fixture inputs and on this repo's synthetic edge-case FASTQs; every output file
 must be byte-identical (gz outputs are compared after decompression).  The flat CLI takes its argument parser, adapter
 table and policy functions from the reference package itself; only the data path differs (porechop_b200/fastq.py).
-The oracle stands in for the engine (tests only).  Skipped where /root/reference does not exist (the GPU box)."""
+The oracle stands in for the engine (tests only).  Skipped without a Porechop checkout (helpers.porechop_checkout)."""
 import contextlib
 import gzip
 import io

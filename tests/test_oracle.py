@@ -1,8 +1,7 @@
 """Pin the oracle (oracle/overlap_oracle.c) to the reference: SURVEY section-4 golden strings, the committed
-golden fixtures (outputs of the unmodified reference C++), and -- when oracle/_ref exists -- the live reference."""
+golden fixtures (outputs of the unmodified reference C++), and the reference's stored strings for seeded random inputs
+(checked against the live reference too when oracle/_ref exists)."""
 import random
-
-import pytest
 
 from helpers import abi_string, load_golden, oracle_lib, oracle_record, oracle_string, ref_lib
 
@@ -95,10 +94,11 @@ def test_record_matches_string():
         assert record_string(oracle_record(rd, ad, sc)) == exp
 
 
-@pytest.mark.skipif(ref_lib() is None, reason='oracle/_ref/cpp_functions.so not built (reference sources absent)')
-def test_live_against_reference():
+def live_cases():
+    """1500 seeded (read, adapter, scoring) inputs; tests/golden/golden_live.json holds the reference's strings for them."""
     rng = random.Random(99)
     schemes = [[3, -6, -5, -2], [3, -6, -2, -2], [2, -3, -2, -5], [1, 0, -1, -1], [4, -5, -3, -3]]
+    out = []
     for _ in range(1500):
         al = rng.choice(['AC', 'ACGT', 'ACGTN'])
         ad = ''.join(rng.choice(al) for _ in range(rng.randint(1, 60)))
@@ -106,5 +106,16 @@ def test_live_against_reference():
         if rng.random() < 0.6:
             p = rng.randint(0, len(rd))
             rd = rd[:p] + ad[rng.randint(0, len(ad) // 2):] + rd[p:]
-        sc = rng.choice(schemes)
-        assert abi_string(oracle_lib(), rd, ad, sc) == abi_string(ref_lib(), rd, ad, sc)
+        out.append((rd, ad, rng.choice(schemes)))
+    return out
+
+
+def test_live_against_reference():
+    """The oracle against the reference C++ on live_cases(): its stored strings, and the library itself when built."""
+    g = load_golden('golden_live.json')
+    cases = live_cases()
+    assert len(g['results']) == len(cases)
+    for (rd, ad, sc), exp in zip(cases, g['results']):
+        assert abi_string(oracle_lib(), rd, ad, sc) == exp
+        if ref_lib() is not None:
+            assert abi_string(ref_lib(), rd, ad, sc) == exp

@@ -1,6 +1,6 @@
 """CPU tier (authoring container only): the run-time drop-in `porechop_b200.patch` under the UNMODIFIED reference CLI.
 
-The reference's own `main()` (porechop/porechop.py:33-79, imported from /root/reference) runs its fixture inputs twice:
+The reference's own `main()` (porechop/porechop.py:33-79, imported from a Porechop checkout) runs its fixture inputs twice:
   baseline  its per-call path on the reference C++ (oracle/_ref/cpp_functions.so),
   patched   with `patch.install()`: one prefetch batch per phase, the original drivers unchanged.
 Everything the CLI writes -- stdout (progress, verbose alignments, summaries) and every output file -- must be
@@ -8,7 +8,7 @@ byte-identical, and the patched run must not have fallen through to a per-call a
 
 There is no GPU in this tier, so the engine's two entry points are replaced by the oracle for the duration of the
 test (the oracle as checker, tests only); the same comparison against the real engine is tests/test_gpu_phases.py's
-job through the golden vectors.  Skipped where /root/reference does not exist (the GPU box).
+job through the golden vectors.  Skipped without a Porechop checkout.
 """
 import contextlib
 import ctypes
@@ -21,12 +21,12 @@ import warnings
 import numpy as np
 import pytest
 
-from helpers import ROOT, oracle_batch, oracle_string
+from helpers import PORECHOP_CHECKOUT, ROOT, oracle_batch, oracle_string
 
-REF = '/root/reference'
+REF = PORECHOP_CHECKOUT
 REF_SO = os.path.join(ROOT, 'oracle', '_ref', 'cpp_functions.so')
-pytestmark = pytest.mark.skipif(not (os.path.isdir(os.path.join(REF, 'porechop')) and os.path.exists(REF_SO)),
-                                reason='needs the reference checkout and oracle/_ref (authoring container)')
+pytestmark = pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, 'porechop')) and os.path.exists(REF_SO)),
+                                reason='needs a Porechop checkout (helpers.porechop_checkout) and oracle/_ref built from it')
 
 
 def load_reference():

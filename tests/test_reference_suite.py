@@ -1,4 +1,4 @@
-"""CPU tier (authoring container only): the REFERENCE'S OWN unittest suite (/root/reference/test/*.py, 85 CLI-level
+"""CPU tier (with a Porechop checkout only): the REFERENCE'S OWN unittest suite (<checkout>/test/*.py, 85 CLI-level
 tests -- SURVEY.md section 4) run against the two drop-ins, with the reference CLI on its own C++ as the baseline
 (tests/refsuite/run_reference_suite.py).  The engine under the drop-ins is the product's own engine.cu + kernels.cuh in the
 host simulation of tests/sim (`--engine sim`; `--engine oracle` uses the C restatement instead, `--engine cuda` the real
@@ -14,12 +14,12 @@ import sys
 
 import pytest
 
-from helpers import ROOT
+from helpers import PORECHOP_CHECKOUT, ROOT
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not (os.path.isdir(os.path.join(REF, 'test')) and
+REF = PORECHOP_CHECKOUT
+pytestmark = pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, 'test')) and
                                      os.path.exists(os.path.join(ROOT, 'oracle', '_ref', 'cpp_functions.so'))),
-                                reason='needs the reference checkout and oracle/_ref (authoring container)')
+                                reason='needs a Porechop checkout (helpers.porechop_checkout) and oracle/_ref built from it')
 
 # tests whose assertions include text of the reference's progress report (adapter table, "N / M reads ...", barcode table)
 REPORT_TESTS = {

@@ -13,7 +13,7 @@ import sys
 import numpy as np
 import pytest
 
-from helpers import DEFAULT, ROOT, load_golden, oracle_batch
+from helpers import DEFAULT, PORECHOP_CHECKOUT, ROOT, load_golden, oracle_batch
 from test_oracle import SURVEY_EDGE, rebuild_fullread_inputs
 
 sys.path.insert(0, os.path.join(ROOT, 'tests', 'sim'))
@@ -335,7 +335,8 @@ def _sim_as_engine(W):
     return install
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/porechop'), reason='needs the reference checkout (authoring container)')
+@pytest.mark.skipif(not (PORECHOP_CHECKOUT and os.path.isdir(os.path.join(PORECHOP_CHECKOUT, 'porechop'))),
+                    reason='needs a Porechop checkout (helpers.porechop_checkout)')
 def test_sim_engine_under_the_unmodified_cli_and_the_flat_cli(W, monkeypatch, tmp_path):
     """tests/test_patch_cli.py and tests/test_flat_cli.py compare the drop-ins with the reference CLI byte for byte, with the
     oracle standing in for the engine; here the same comparisons run on the product's engine code (host simulation): the
